@@ -2,6 +2,7 @@
 """bench.py -- registrations/sec of the VGICP hot path on B200 (BASELINE.json metric), one JSON line on stdout.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c2_direct1|c3|c4|c4_direct1|c5]
+                    [--dump-outputs DIR]
 
 Workload (N=1 default, BASELINE configs[1]): the reference's benchmark pair (tests/golden/pair_0p1.npz = data/251370668.pcd
 vs 251371071.pcd after align.cpp's filter + ApproximateVoxelGrid(0.1): 17047 / 17334 points), FastVGICPCuda, DIRECT27,
@@ -28,6 +29,14 @@ saturates at 8 streams).  Host threads are pinned to the cores of the GPU's NUMA
   c4     : BASELINE config 4, the 1M-point pair: stage times and the evaluation kernel's HBM roofline (DIRECT27 and DIRECT1) on one
            GPU; with N > 1 the same registration with stage 1 and stage 3 sharded over the N ranks (in-kernel NVLink exchanges),
            speed-up against the unsharded registration measured in the same run, agreement and bit-identity across ranks.
+
+--dump-outputs DIR (rank 0): what the timed registrations of the last step returned, one registration per stream, as DIR/<name>.npy
+(float64 unless noted; the inputs are the same from run to run, so two builds can be compared output for output):
+  pose, hessian       (S,4,4), (S,6,6): final transformation and Hessian of the resident arm (vgicp_register)
+  counters            (S,5): nr_iterations, converged, n_linearize, n_compute_error, lm_failed of the same registrations
+  e2e_pose            (S,4,4): final transformation of the e2e arm
+  e2e_aligned         (S,n,3) float32: the aligned source clouds the e2e arm read back; above 16 MB a fixed seeded sample of n rows,
+                      the same for every stream, whose indices are in e2e_aligned_rows (n,)
 
 N>1 (torchrun): the 17k-pt path does not shard usefully (SURVEY 8e) -> replicas, S registration streams per GPU, no
 data-path collective; value = N*S*K registrations / max-over-ranks time ("weak" scaling).  The c4 record is the sharded path.
@@ -399,6 +408,19 @@ def c4_record(torch, dev, local_rank, rank, world, peak_gbs, note):
     return rec
 
 
+def write_outputs(out_dir, arrays, aligned_budget=16 << 20):
+    """--dump-outputs: every array as out_dir/<name>.npy; the aligned clouds above `aligned_budget` bytes as a fixed, seeded sample of
+    rows (the same rows for every stream) so that the files stay small at the 1M-point workloads."""
+    os.makedirs(out_dir, exist_ok=True)
+    a = arrays.get("e2e_aligned")
+    if a is not None and a.nbytes > aligned_budget:
+        n = a.shape[1]
+        rows = np.sort(np.random.default_rng(0).choice(n, size=aligned_budget // (a.shape[0] * 12), replace=False))
+        arrays["e2e_aligned"], arrays["e2e_aligned_rows"] = a[:, rows], rows.astype(np.float64)
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v)
+
+
 # -------------------------------------------------------------------------------------------------------- GPU arm
 def main():
     # stdout carries exactly one JSON line: route everything else that writes to fd 1 (NCCL's version banner, library
@@ -423,6 +445,7 @@ def main():
                          "leave the host cores of a NUMA node to the ranks that share it)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-c4", action="store_true", help="skip the 1M-point sub-record (config 4: evaluation roofline at N=1, sharded registration at N>1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (see the module docstring)")
     ap.add_argument("--e2e-impl", default="class", choices=["class", "batch"],
                     help="end-to-end arm: the FastVGICPCuda class from S Python threads (default, verified), or one vgicp_batch_register C call per timed region "
                          "(include/vgicp_batch_b200.h; not yet verified on hardware)")
@@ -544,7 +567,7 @@ def main():
 
     def run_streams(step_fn, stream_list, steps):
         """`steps` registrations on each of the S streams (one host thread + one handle per stream), distinct pairs from the
-        pool; returns (device time from the common start event to the last stream's end event [ms], last result)."""
+        pool; returns (device time from the common start event to the last stream's end event [ms], last result of every stream)."""
         start = torch.cuda.Event(enable_timing=True)
         ends = [torch.cuda.Event(enable_timing=True) for _ in range(S)]
         out = [None] * S
@@ -566,7 +589,7 @@ def main():
         for t_ in th:
             t_.join()
         torch.cuda.synchronize()
-        return max(start.elapsed_time(e) for e in ends), out[0]
+        return max(start.elapsed_time(e) for e in ends), out
 
     # ---- value: resident inputs, S concurrent streams
     note("handles ready")
@@ -576,10 +599,15 @@ def main():
     sampler = ClockSampler(local_rank) if rank == 0 else None
     l0 = sum(c.launch_count() for c in cores)
     t_wall0 = time.perf_counter()
-    total_ms, res = run_streams(step_resident, streams, K)
+    total_ms, last = run_streams(step_resident, streams, K)
     barrier()
     wall_s = time.perf_counter() - t_wall0
     launches = sum(c.launch_count() for c in cores) - l0
+    res = last[0]
+    dump = {}
+    if args.dump_outputs:
+        dump["pose"] = np.stack([pose_from_c(r.T) for r in last])
+        dump["hessian"] = np.stack([np.array(r.H).reshape(6, 6).T for r in last])
 
     # ---- e2e: host buffers through the reference-facing class, S concurrent streams
     note("value arm done")
@@ -602,20 +630,28 @@ def main():
             res_b = call(20, REG_PLANE)
             ev1.record()
             torch.cuda.synchronize()
-            return ev0.elapsed_time(ev1), pose_from_c(res_b[0].T)
+            return ev0.elapsed_time(ev1), res_b
 
         run_batch(W)
         barrier()
-        total_ms_e2e, T_e2e = run_batch(K)
+        total_ms_e2e, last_e2e = run_batch(K)
         barrier()
+        T_e2e = pose_from_c(last_e2e[0].T)
+        if args.dump_outputs:  # the last S registrations of the call are the last step's
+            dump["e2e_pose"] = np.stack([pose_from_c(r.T) for r in last_e2e[-S:]])
+            dump["e2e_aligned"] = np.stack(aligned_all[S * K - S:S * K])
         launches_e2e = int(launches)  # the pool's handles are internal: same launches per registration as the resident arm
         e2e_api = "vgicp_batch_register (one C call for all registrations of the timed region; pinned host buffers, aligned clouds + poses read back)"
     else:
         run_streams(step_e2e, e2e_streams, W)
         barrier()
         l1 = sum(r.vgicp_cuda_.launch_count() for r in regs)
-        total_ms_e2e, T_e2e = run_streams(step_e2e, e2e_streams, K)
+        total_ms_e2e, last_e2e = run_streams(step_e2e, e2e_streams, K)
         barrier()
+        T_e2e = last_e2e[0]
+        if args.dump_outputs:
+            dump["e2e_pose"] = np.stack(last_e2e).astype(np.float64)
+            dump["e2e_aligned"] = np.stack([a.numpy() for a in aligned_h])
         launches_e2e = sum(r.vgicp_cuda_.launch_count() for r in regs) - l1
     clocks = sampler.stop() if sampler else None
 
@@ -809,6 +845,9 @@ def main():
         "wall_ms_per_step": 1e3 * wall_s / K, "host_placement": placement, "c4": c4, "published_configurations": extras,
         "pose_check": {"translation": [float(x) for x in T_val[:3, 3]], "e2e_vs_resident_max_abs": float(np.abs(np.asarray(T_e2e, dtype=np.float64) - T_val).max())},
     }
+    if args.dump_outputs:
+        dump["counters"] = np.array([[r.nr_iterations, r.converged, r.n_linearize, r.n_compute_error, r.lm_failed] for r in last], dtype=np.float64)
+        write_outputs(args.dump_outputs, dump)
     print(json.dumps(line), file=_REAL_STDOUT, flush=True)
     D.finalize()
 

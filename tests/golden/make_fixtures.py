@@ -1,15 +1,15 @@
 #!/usr/bin/env python3
 """Generate the committed golden input fixtures from the reference's own data files.
 
-Run in the build container only (needs /root/reference, which does not exist on the GPU box):
+    python tests/golden/make_fixtures.py <fast_gicp checkout>/data
 
-    python tests/golden/make_fixtures.py
-
-Reads  /root/reference/data/251370668.pcd (target), 251371071.pcd (source), relative.txt
+Reads  <data>/251370668.pcd (target), 251371071.pcd (source), relative.txt
 Writes tests/golden/pair_0p1.npz   -- the reference's benchmark inputs: near-origin filter
                                       (src/align.cpp:128-133) + ApproximateVoxelGrid(0.1) (src/align.cpp:136-147)
        tests/golden/pair_0p2.npz   -- the reference's test inputs: VoxelGrid(0.2) (src/test/gicp_test.cpp:55-65)
        tests/golden/relative.txt   -- ground-truth pose (data/relative.txt), numbers only
+       tests/golden/scan_window.npz -- a window of SCAN_WINDOW raw points of each scan and its ApproximateVoxelGrid(0.1) without
+                                      and with the near-origin filter (the raw scans are too large to commit whole)
 
 PCL is not vendored in the reference, so both filters are restated from the published PCL algorithm
 (pcl/filters/approximate_voxel_grid.hpp, voxel_grid.hpp).  The restatement of ApproximateVoxelGrid (and of the PCD reader) is PINNED by
@@ -21,8 +21,9 @@ import os
 import sys
 import numpy as np
 
-REF = "/root/reference/data"
 OUT = os.path.dirname(os.path.abspath(__file__))
+# raw points [start, start + 3072) of each scan: a stretch of the scan with many invalid returns at the origin
+SCAN_WINDOW = slice(36864, 36864 + 3072)
 
 
 def read_pcd_xyz(path):
@@ -118,13 +119,11 @@ def voxel_grid(pts, leaf):
     return out
 
 
-def main():
-    if not os.path.isdir(REF):
-        sys.exit("needs /root/reference/data (build container only)")
-    tgt = read_pcd_xyz(os.path.join(REF, "251370668.pcd"))
-    src = read_pcd_xyz(os.path.join(REF, "251371071.pcd"))
+def main(ref):
+    tgt = read_pcd_xyz(os.path.join(ref, "251370668.pcd"))
+    src = read_pcd_xyz(os.path.join(ref, "251371071.pcd"))
     assert tgt.shape == (69088, 3) and src.shape == (69792, 3)
-    rel = np.loadtxt(os.path.join(REF, "relative.txt"))
+    rel = np.loadtxt(os.path.join(ref, "relative.txt"))
     np.savetxt(os.path.join(OUT, "relative.txt"), rel, fmt="%.9g")
 
     # benchmark protocol (align.cpp): filter + ApproximateVoxelGrid(0.1)
@@ -145,6 +144,18 @@ def main():
     print("pair_0p2: target", len(t2), "source", len(s2))
     np.savez_compressed(os.path.join(OUT, "pair_0p2.npz"), target=t2, source=s2)
 
+    win = {}
+    for name, cloud in (("target", tgt), ("source", src)):
+        raw = np.ascontiguousarray(cloud[SCAN_WINDOW])
+        win[name + "_raw"] = raw
+        win[name + "_avg"] = approximate_voxel_grid(raw, 0.1)
+        win[name + "_avg_filtered"] = approximate_voxel_grid(remove_near_origin(raw), 0.1)
+    print("scan_window: raw", len(win["target_raw"]), "/", len(win["source_raw"]), "-> target", len(win["target_avg"]), len(win["target_avg_filtered"]),
+          "source", len(win["source_avg"]), len(win["source_avg_filtered"]))
+    np.savez_compressed(os.path.join(OUT, "scan_window.npz"), **win)
+
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2 or not os.path.isdir(sys.argv[1]):
+        sys.exit(__doc__)
+    main(sys.argv[1])

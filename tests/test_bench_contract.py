@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -42,3 +44,22 @@ def test_gpu_arm_refuses_to_run_without_a_device():
         return
     r = run_bench([])
     assert r.stdout.strip() == "" and "no CPU fallback" in (r.stderr + r.stdout)
+
+
+def test_dump_outputs_keep_small_arrays_and_sample_large_clouds(tmp_path):
+    """--dump-outputs: small arrays are written as they are; aligned clouds above the budget become the same seeded rows of every
+    stream, with the row indices beside them, identical from run to run."""
+    import bench
+
+    pose = np.arange(32, dtype=np.float64).reshape(2, 4, 4)
+    cloud = np.random.default_rng(3).random((2, 50000, 3), dtype=np.float32)
+    for d in ("a", "b"):
+        bench.write_outputs(str(tmp_path / d), {"pose": pose, "e2e_aligned": cloud}, aligned_budget=120000)
+    assert sorted(os.listdir(tmp_path / "a")) == ["e2e_aligned.npy", "e2e_aligned_rows.npy", "pose.npy"]
+    assert np.array_equal(np.load(tmp_path / "a" / "pose.npy"), pose)
+    got, rows = np.load(tmp_path / "a" / "e2e_aligned.npy"), np.load(tmp_path / "a" / "e2e_aligned_rows.npy")
+    assert got.dtype == np.float32 and rows.dtype == np.float64 and got.nbytes <= 120000 and got.shape == (2, len(rows), 3)
+    assert len(np.unique(rows)) == len(rows) and np.array_equal(got, cloud[:, rows.astype(np.int64)])
+    assert np.array_equal(np.load(tmp_path / "b" / "e2e_aligned.npy"), got)
+    bench.write_outputs(str(tmp_path / "c"), {"e2e_aligned": cloud[:, :100]}, aligned_budget=120000)
+    assert sorted(os.listdir(tmp_path / "c")) == ["e2e_aligned.npy"] and np.array_equal(np.load(tmp_path / "c" / "e2e_aligned.npy"), cloud[:, :100])
